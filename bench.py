@@ -2,6 +2,7 @@
 """bench.py -- throughput of the MonoDETR hot path on B200 (see DESIGN.md "Measurement").
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload model|msda|infer]
+                    [--dump-outputs DIR]
 
 Prints ONE JSON line (rank 0).  Workloads:
   model : full MonoDETR forward+backward, ResNet-50, 1280x384 synthetic images, train mode
@@ -10,6 +11,8 @@ Prints ONE JSON line (rank 0).  Workloads:
           8 heads x 32 ch, 4 points) -- BASELINE.json configs[1] family
 `--impl reference` times the reference's CPU implementation of the same workload (the oracle port; the
 Python reference itself cannot travel to the GPU box) on all host cores, rank 0 only.
+`--dump-outputs DIR` (b200 arm, rank 0) writes what the last timed step computed as DIR/<name>.npy (see dump_outputs), so
+that two builds run with the same arguments -- hence the same seeded inputs and weights -- can be compared output for output.
 """
 import argparse
 import json
@@ -19,6 +22,7 @@ import subprocess
 import sys
 import tempfile
 import time
+import zlib
 
 import torch
 
@@ -87,6 +91,32 @@ class ClockSampler:
         if sm:
             out.update(sm_mhz=statistics.median(sm), sm_max_mhz=max(mx), reasons=sorted(reasons), samples=len(sm))
         return out
+
+
+DUMP_LIMIT_BYTES = 64 * 1024 * 1024
+
+
+def sampled(t, k, name):
+    """`t` itself if it has at most k elements, else k of its (flattened) elements at fixed positions: the first k of a
+    permutation seeded by crc32(name), in ascending order.  The same name and shape always select the same elements."""
+    if t.numel() <= k:
+        return t
+    g = torch.Generator().manual_seed(zlib.crc32(name.encode()))
+    idx = torch.randperm(t.numel(), generator=g)[:k].sort().values
+    return t.detach().reshape(-1)[idx.to(t.device)]
+
+
+def dump_outputs(path, arrays):
+    """Write every tensor of `arrays` (name -> tensor) as path/<name>.npy: float64 tensors as float64, all others as float32.
+    Refuses to write more than DUMP_LIMIT_BYTES in all."""
+    import numpy as np
+    host = {n: t.detach().to("cpu", torch.float64 if t.dtype == torch.float64 else torch.float32) for n, t in arrays.items()}
+    total = sum(t.numel() * t.element_size() for t in host.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(path, exist_ok=True)
+    for n, t in host.items():
+        np.save(os.path.join(path, n + ".npy"), t.numpy())
 
 
 def dist_info():
@@ -163,14 +193,19 @@ def run_msda_b200(args, rank, local_rank, ws):
     evs = [[torch.cuda.Event(enable_timing=True) for _ in range(3)] for _ in range(args.steps)]
     lc0 = _lib.launch_count()
     for i in range(args.steps):
+        grads = None                 # released before the step allocates, as when the step discards them
         flush.zero_()
         evs[i][0].record()
         out = ms_deform_attn_forward(*dv[:5], 64)
         evs[i][1].record()
-        ms_deform_attn_backward(*dv[:5], dv[5], 64)
+        grads = ms_deform_attn_backward(*dv[:5], dv[5], 64)
         evs[i][2].record()
     barrier()
     launches = _lib.launch_count() - lc0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {n: sampled(t, 1 << 21, n) for n, t in
+                                         zip(("out", "grad_value", "grad_loc", "grad_attn"), (out,) + tuple(grads))})
+    del grads
     clocks = sampler.stop() if sampler else None
     t_fwd = [evs[i][0].elapsed_time(evs[i][1]) for i in range(args.steps)]
     t_bwd = [evs[i][1].elapsed_time(evs[i][2]) for i in range(args.steps)]
@@ -336,7 +371,14 @@ def main():
     ap.add_argument("--batch", type=int, default=0, help="per-GPU batch (default: 8 at N=1, 16 at N>1 for model)")
     ap.add_argument("--lq", type=int, default=10200)
     ap.add_argument("--uniform-loc", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="b200 arm: write the results of the last timed step as DIR/<name>.npy (float32/float64, <= 64 MiB; "
+                         "arrays above a size cap as a fixed seeded sample)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     rank, local_rank, ws = dist_info()
 
@@ -358,7 +400,8 @@ def main():
     else:
         from monodetr_b200 import bench_model
         quick = bool(os.environ.get("MDB_BENCH_QUICK"))      # A/B runs: the timed step and e2e only (no probes, batch-16 point, CPU arm, extras)
-        line = bench_model.run(args, rank, local_rank, ws, infer=(args.workload == "infer"), extras=not quick)
+        line = bench_model.run(args, rank, local_rank, ws, infer=(args.workload == "infer"), extras=not quick,
+                               dump_dir=args.dump_outputs)
         if line is not None and ws == 1 and args.workload == "model" and not quick:
             if not args.batch and not os.environ.get("MDB_BENCH_NO_B16"):
                 # the N > 1 runs use batch 16 per GPU (BASELINE configs[3]): the like-for-like single-GPU point for scaling

@@ -95,9 +95,10 @@ def gemm_probe(dev, flush):
     return out
 
 
-def run(args, rank, local_rank, ws, infer=False, batch_override=None, extras=True):
+def run(args, rank, local_rank, ws, infer=False, batch_override=None, extras=True, dump_dir=None):
     """infer=False: BASELINE configs[2]/[3] (train step).  infer=True: configs[4], eval-mode forward only, batch 32,
-    no gradients, N>1 = independent replicas (no collective)."""
+    no gradients, N>1 = independent replicas (no collective).  dump_dir: rank 0 writes the last timed step's results there
+    (bench.dump_outputs): the surrogate loss, every output head, and (train) every parameter gradient."""
     dev = torch.device("cuda", local_rank)
     torch.cuda.set_device(dev)
     B = batch_override or args.batch or (32 if infer else (8 if ws == 1 else 16))
@@ -115,17 +116,22 @@ def run(args, rank, local_rank, ws, infer=False, batch_override=None, extras=Tru
     loss_buf = torch.zeros((), device=dev)
     loss_host = torch.zeros(()).pin_memory()
 
+    last = {}      # the latest call's outputs; in graph mode the captured tensors, which every replay rewrites
+
     def fwd_bwd():
+        last.clear()
         if infer:
             with torch.no_grad():
                 out = model(images, calibs, None, sizes)
                 loss_buf.copy_(surrogate_loss(out))          # checksum over every output head = the step's result
+            last["out"] = out
             return
         bucket.zero()
         out = model(images, calibs, None, sizes)
         loss = surrogate_loss(out)
         loss.backward()
         loss_buf.copy_(loss.detach())
+        last["out"] = out
 
     def barrier():
         if ws > 1:
@@ -191,6 +197,17 @@ def run(args, rank, local_rank, ws, infer=False, batch_override=None, extras=Tru
     if ws > 1:
         dist.all_reduce(tt, op=dist.ReduceOp.MAX)
     total_ms = float(tt.item())
+    if dump_dir is not None and rank == 0:
+        from bench import dump_outputs, sampled
+        arrays = {"loss": loss_buf}
+        for k, v in last["out"].items():
+            for name, t in ([(f"out.aux{i}.{kk}", vv) for i, aux in enumerate(v) for kk, vv in aux.items()] if k == "aux_outputs"
+                            else [(f"out.{k}", v)]):
+                arrays[name] = sampled(t, 1 << 21, name)
+        for n, p in model.named_parameters():
+            if p.grad is not None:
+                arrays[f"grad.{n}"] = sampled(p.grad, 1 << 14, f"grad.{n}")
+        dump_outputs(dump_dir, arrays)
 
     # ---- exposed all-reduce (N > 1): the flat-bucket pack + ncclAllReduce + divide run after the graph replay, not overlapped
     allreduce_ms = None

@@ -576,9 +576,13 @@ class _Stream:
 
 def install(monkeypatch, precision=1):
     """Route the product's host code to the fake library and give it a dummy CUDA stream API (test-scoped)."""
-    from monodetr_b200 import _lib
+    from monodetr_b200 import _lib, functional, tc
     fake = FakeLib(precision)
     monkeypatch.setattr(_lib, "_lib", fake)
+    # per-process caches that GPU tests run earlier in the same session fill with real CUDA streams / device buffers
+    monkeypatch.setattr(functional, "_SIDE_STREAMS", {})
+    monkeypatch.setattr(functional, "_BRANCH_STREAMS", {})
+    monkeypatch.setattr(tc, "_WORKSPACE", {})
     stream = _Stream()
     monkeypatch.setattr(torch.cuda, "current_stream", lambda *a, **k: stream)
     monkeypatch.setattr(torch.cuda, "Stream", _Stream)

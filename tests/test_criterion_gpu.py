@@ -7,6 +7,7 @@ import pytest
 import torch
 
 from oracle import criterion as oc
+from test_oracle_criterion import assert_grad_matches_golden
 
 pytestmark = pytest.mark.gpu
 GOLD = np.load(os.path.join(os.path.dirname(__file__), "golden", "criterion.npz"))
@@ -75,9 +76,8 @@ def test_against_reference_golden(name):
         for k, t in d.items():
             if not torch.is_tensor(t) or k.startswith("_"):
                 continue
-            g = GOLD[f"{name}.grad.{layer}.{k}"]
-            got = t.grad.cpu().numpy() if t.grad is not None else np.zeros_like(g)
-            np.testing.assert_allclose(got, g, rtol=2e-4, atol=1e-9 + 2e-5 * np.abs(g).max(), err_msg=f"{layer}.{k}")
+            got = t.grad.cpu().numpy() if t.grad is not None else np.zeros(tuple(t.shape), np.float32)
+            assert_grad_matches_golden(got, f"{name}.grad.{layer}.{k}", rtol=2e-4, atol_rel=2e-5)
 
 
 @pytest.mark.parametrize("seed,B,Q,training,kw", [(31, 8, 550, True, {}), (32, 5, 50, False, {}), (33, 2, 550, True, {"max_gt": 50}),

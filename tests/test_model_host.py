@@ -1,7 +1,9 @@
 """CPU: host-side contract of the product model (no compute): state_dict keys/shapes equal the reference's,
 trainability rule, aliasing, and that the forward fails loudly without CUDA (no CPU fallback)."""
+import json
 import os
 import sys
+import types
 
 import pytest
 import torch
@@ -63,39 +65,42 @@ def test_forward_requires_cuda(model):
         model(images, calibs, None, sizes)
 
 
-@pytest.mark.reference
+def _reference_spec():
+    with open(os.path.join(ROOT, "tests", "golden", "reference_model_spec.json")) as f:
+        return json.load(f)
+
+
 def test_state_dict_matches_unmodified_reference(model):
-    sys.path.insert(0, os.path.join(ROOT, "tools"))
-    import warnings
-    warnings.filterwarnings("ignore")
-    import ref_shims
-    pkg = ref_shims.install()
-    ref, _ = pkg.build_monodetr(ref_shims.load_cfg()["model"])
-    a = {k: tuple(v.shape) for k, v in ref.state_dict().items()}
-    b = {k: tuple(v.shape) for k, v in model.state_dict().items()}
-    assert a == b
-    assert list(ref.state_dict().keys()) == list(model.state_dict().keys()) or set(a) == set(b)
-    ref_train = {n for n, p in ref.named_parameters() if p.requires_grad}
-    mine_train = {n for n, p in model.named_parameters() if p.requires_grad}
-    assert ref_train == mine_train
+    spec = _reference_spec()
+    assert [k for k, _ in spec["state_dict"]] == list(model.state_dict().keys())
+    assert {k: tuple(s) for k, s in spec["state_dict"]} == {k: tuple(v.shape) for k, v in model.state_dict().items()}
+    assert set(spec["trainable"]) == {n for n, p in model.named_parameters() if p.requires_grad}
 
 
-@pytest.mark.reference
-def test_build_returns_the_reference_criterion_when_importable():
+def test_build_returns_the_reference_criterion_when_importable(monkeypatch):
     """B2: build_monodetr(cfg) -> (model, criterion) like monodetr.py:550-614; with the reference package importable
-    (as inside tools/train_val.py) the criterion is the reference's SetCriterion with the reference's weight_dict."""
-    sys.path.insert(0, os.path.join(ROOT, "tools"))
-    import warnings
-    warnings.filterwarnings("ignore")
-    import ref_shims
-    pkg = ref_shims.install()
-    cfg = ref_shims.load_cfg()["model"]
-    _, ref_crit = pkg.build_monodetr(cfg)
-    from monodetr_b200 import build_monodetr
+    (as inside tools/train_val.py) the criterion is the reference's SetCriterion, built with what the reference's build()
+    passes it (stored in tests/golden/reference_model_spec.json).  A stand-in `lib.models.monodetr` records the call."""
+    spec = _reference_spec()
+    cfg = spec["model_cfg"]
+
+    class SetCriterion(torch.nn.Module):
+        def __init__(self, num_classes, matcher, weight_dict, focal_alpha, losses):
+            super().__init__()
+            self.num_classes, self.matcher, self.weight_dict, self.focal_alpha, self.losses = \
+                num_classes, matcher, weight_dict, focal_alpha, losses
+
+    matcher = object()
+    pkg = {name: types.ModuleType(name) for name in ("lib", "lib.models", "lib.models.monodetr",
+                                                      "lib.models.monodetr.matcher", "lib.models.monodetr.monodetr")}
+    pkg["lib.models.monodetr.matcher"].build_matcher = lambda c: matcher if c == cfg else None
+    pkg["lib.models.monodetr.monodetr"].SetCriterion = SetCriterion
+    for name, mod in pkg.items():
+        monkeypatch.setitem(sys.modules, name, mod)
     _, crit = build_monodetr(cfg)
-    assert type(crit) is type(ref_crit)
-    assert crit.weight_dict == ref_crit.weight_dict and crit.losses == ref_crit.losses
-    assert crit.focal_alpha == ref_crit.focal_alpha and crit.num_classes == ref_crit.num_classes
+    assert type(crit) is SetCriterion and crit.matcher is matcher
+    ref = spec["criterion"]
+    assert crit.weight_dict == ref["weight_dict"] and crit.losses == ref["losses"]
+    assert crit.focal_alpha == ref["focal_alpha"] and crit.num_classes == ref["num_classes"]
     # without loss weights in the cfg (stand-alone model use) there is nothing to build a criterion from
-    from monodetr_b200.monodetr import DEFAULT_MODEL_CFG
     assert build_monodetr(DEFAULT_MODEL_CFG)[1] is None

@@ -1,8 +1,7 @@
-"""Pin oracle/monodetr_torch.py (CPU restatement of the model path) against the UNMODIFIED reference imported
-from /root/reference (authoring container only: marker `reference`) and against the committed fixture
-tests/golden/model_eval_small.npz (everywhere).  CPU only."""
+"""Pin oracle/monodetr_torch.py (CPU restatement of the model path) against outputs of the UNMODIFIED reference, stored by
+tools/gen_golden_reference_pins.py and tools/gen_golden_model.py under tests/golden/.  CPU only."""
+import json
 import os
-import sys
 
 import numpy as np
 import pytest
@@ -10,87 +9,65 @@ import torch
 
 from oracle import monodetr_torch as om
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-sys.path.insert(0, os.path.join(ROOT, "tools"))
-
 OUT_KEYS = ("pred_logits", "pred_boxes", "pred_3d_dim", "pred_depth", "pred_angle", "pred_depth_map_logits")
 
 
-def _build_reference(dropout):
-    import warnings
-    warnings.filterwarnings("ignore")
-    import ref_shims
-    pkg = ref_shims.install()
-    cfg = ref_shims.load_cfg()["model"]
-    cfg["dropout"] = dropout
-    torch.manual_seed(0)
-    model, _ = pkg.build_monodetr(cfg)
-    if dropout == 0.0:
-        # the depth encoder hard-codes dropout=0.1 (depth_predictor.py:49-50): neutralise every dropout in memory
-        for m in model.modules():
-            if isinstance(m, torch.nn.Dropout):
-                m.p = 0.0
-            if isinstance(m, torch.nn.MultiheadAttention):
-                m.dropout = 0.0
-    return model
-
-
-@pytest.mark.reference
-def test_state_dict_spec_matches_reference():
-    model = _build_reference(0.1)
-    ref = {k: tuple(v.shape) for k, v in model.state_dict().items()}
+def test_state_dict_spec_matches_reference(golden_dir):
+    with open(os.path.join(golden_dir, "reference_model_spec.json")) as f:
+        ref = {k: tuple(s) for k, s in json.load(f)["state_dict"]}
     mine = {k: tuple(v.shape) for k, v in om.with_aliases({k: torch.empty(s) for k, s in om.state_dict_spec().items()}).items()}
     assert ref == mine
     assert len(ref) == 582
 
 
-@pytest.mark.reference
 @pytest.mark.parametrize("training", [False, True])
-def test_oracle_forward_matches_reference(training):
-    model = _build_reference(0.0)
-    sd = {k: v.detach().clone() for k, v in model.state_dict().items()}
-    # perturb the zero-initialised MSDA projections so every code path carries signal
-    g = torch.Generator().manual_seed(1)
-    for k in sd:
-        if k.endswith("sampling_offsets.weight") or k.endswith("attention_weights.weight"):
-            sd[k] = torch.randn(sd[k].shape, generator=g) * 0.02
-    model.load_state_dict(sd)
-    model.train(training)
-    images, calibs, sizes = om.synthetic_inputs(1, 0, H=192, W=640)
+def test_oracle_forward_matches_reference(training, golden_dir):
+    g = np.load(os.path.join(golden_dir, "reference_model_forward.npz"))
+    mode = "train" if training else "eval"
+    sd = om.deterministic_state_dict(base_seed=int(g["base_seed"]))
+    images, calibs, sizes = om.synthetic_inputs(int(g["B"]), int(g["seed"]), H=int(g["H"]), W=int(g["W"]))
     with torch.no_grad():
-        ref = model(images, calibs, None, sizes)
         mine = om.forward(sd, images, calibs, sizes, training=training)
+
+    def close(got, ref, scale, name):
+        # The fixture comes from another machine, whose CPU kernels sum in another fp32 order: the absolute bar scales with
+        # the output's magnitude, as in the other fixture comparisons.
+        np.testing.assert_allclose(got, ref, rtol=2e-4, atol=2e-5 * max(1.0, float(scale)), err_msg=name)
+
     for k in OUT_KEYS:
-        np.testing.assert_allclose(mine[k].numpy(), ref[k].numpy(), rtol=2e-4, atol=2e-5, err_msg=k)
-    for a, b in zip(mine["aux_outputs"], ref["aux_outputs"]):
+        if k == "pred_depth_map_logits":     # stored as a seeded sample of the map
+            scale = g[f"{mode}.{k}.absmax"]
+            close(np.abs(mine[k].numpy()).max(), scale, scale, k + " max")
+            close(mine[k].numpy().reshape(-1)[g[f"{mode}.{k}.idx"]], g[f"{mode}.{k}.val"], scale, k)
+        else:
+            close(mine[k].numpy(), g[f"{mode}.{k}"], np.abs(g[f"{mode}.{k}"]).max(), k)
+    assert len(mine["aux_outputs"]) == 2
+    for i, a in enumerate(mine["aux_outputs"]):
+        assert sorted(a) == sorted(k[len(f"{mode}.aux{i}."):] for k in g.files if k.startswith(f"{mode}.aux{i}."))
         for k in a:
-            np.testing.assert_allclose(a[k].numpy(), b[k].numpy(), rtol=2e-4, atol=2e-5, err_msg="aux " + k)
+            ref = g[f"{mode}.aux{i}.{k}"]
+            close(a[k].numpy(), ref, np.abs(ref).max(), "aux " + k)
 
 
-@pytest.mark.reference
-def test_oracle_gradients_match_reference():
-    model = _build_reference(0.0)
-    sd0 = om.with_aliases(om.deterministic_state_dict())
-    model.load_state_dict(sd0)
-    model.train(True)
-    images, calibs, sizes = om.synthetic_inputs(1, 0, H=96, W=320)
-    om.surrogate_loss(model(images, calibs, None, sizes)).backward()
+def test_oracle_gradients_match_reference(golden_dir):
+    g = np.load(os.path.join(golden_dir, "reference_model_grads.npz"))
+    images, calibs, sizes = om.synthetic_inputs(int(g["B"]), int(g["seed"]), H=int(g["H"]), W=int(g["W"]))
     sd = {k: v.clone().requires_grad_(v.dtype.is_floating_point) for k, v in om.deterministic_state_dict().items()}
     om.surrogate_loss(om.forward(sd, images, calibs, sizes, training=True)).backward()
     # d(bilinear sample)/d(location) is discontinuous at cell borders, so gradients that flow through sampling
     # locations (query_embed, reference_points, sampling_offsets) can differ by O(1e-2) between two fp32
     # evaluation orders; everything else agrees to ~1e-4.  Gradients that are analytically zero (key biases of
-    # a softmax) are skipped.
+    # a softmax) are skipped.  The reference's gradients are stored as max|grad| and a seeded sample that holds the argmax.
     rels = []
-    for name, p in model.named_parameters():
-        if p.grad is None or name not in sd:
-            continue
-        gm = sd[name].grad
+    off = g["offsets"]
+    for i, name in enumerate(g["names"]):
+        gm = sd[str(name)].grad
         assert gm is not None, name
-        scale = float(p.grad.abs().max())
+        scale = float(g["scale"][i])
         if scale < 1e-6:
             continue
-        rel = float((gm - p.grad).abs().max()) / scale
+        gm = gm.numpy().reshape(-1)
+        rel = max(float(np.abs(gm[g["idx"][off[i]:off[i + 1]]] - g["val"][off[i]:off[i + 1]]).max()), abs(float(np.abs(gm).max()) - scale)) / scale
         assert rel <= 5e-2, (name, rel)
         rels.append(rel)
     assert len(rels) > 250

@@ -2,7 +2,9 @@
 HungarianMatcher, lib/models/monodetr/monodetr.py SetCriterion incl. DDNLoss) run on CPU through in-memory shims
 (tools/ref_shims.py + the three below; no reference file is edited):  `Tensor.cuda()` -> identity and `torch.tensor(...,
 device='cuda')` -> CPU, because loss_angles / loss_depth_map hard-code the device (monodetr.py:443,462).
-Run in the build container:  python tools/gen_golden_criterion.py  -> tests/golden/criterion.npz"""
+The gradient of the depth-map logits (a dense B x 81 x 24 x 80 map) is stored as max|grad| and a seeded sample of
+DEPTH_MAP_SAMPLE entries, which keeps the fixture small.
+    python tools/gen_golden_criterion.py  -> tests/golden/criterion.npz"""
 import os
 import sys
 
@@ -21,6 +23,8 @@ _tensor = torch.tensor
 torch.tensor = lambda *a, **k: _tensor(*a, **{kk: vv for kk, vv in k.items() if kk != "device"})
 from lib.models.monodetr.matcher import HungarianMatcher  # noqa: E402
 from lib.models.monodetr.monodetr import SetCriterion  # noqa: E402
+
+DEPTH_MAP_SAMPLE = 4096
 
 matcher = HungarianMatcher(cost_class=2, cost_bbox=5, cost_giou=2, cost_3dcenter=10)
 losses = ["labels", "boxes", "cardinality", "depths", "dims", "angles", "center", "depth_map"]
@@ -51,7 +55,13 @@ for name, (seed, B, Q, training) in CASES.items():
     out[f"{name}.total"] = np.asarray(float(total), np.float64)
     for i, (k, t) in enumerate(leaves):
         layer = "main" if i < 6 else f"aux{(i - 6) // 5}"
-        out[f"{name}.grad.{layer}.{k}"] = t.grad.numpy() if t.grad is not None else np.zeros(t.shape, np.float32)
+        g = t.grad.numpy() if t.grad is not None else np.zeros(t.shape, np.float32)
+        if k == "pred_depth_map_logits":
+            idx = np.sort(np.random.default_rng(seed).choice(g.size, DEPTH_MAP_SAMPLE, replace=False)).astype(np.int64)
+            out[f"{name}.grad.{layer}.{k}.idx"], out[f"{name}.grad.{layer}.{k}.val"] = idx, g.reshape(-1)[idx]
+            out[f"{name}.grad.{layer}.{k}.absmax"] = np.abs(g).max()
+        else:
+            out[f"{name}.grad.{layer}.{k}"] = g
     g = 11 if training else 1
     for l, od in enumerate([o] + o["aux_outputs"]):
         ind = matcher({k: v.detach() for k, v in od.items() if k != "aux_outputs"}, targets, group_num=g)
